@@ -26,6 +26,10 @@ synthetic 1024x1024 pages per GPU (BASELINE.json configs[2]/[3]: batch 16 per GP
 * cpu_baseline / --impl reference: the oracle restatement of the reference's CPU path for the SAME stages
                (oracle/net_ref.py + oracle/postproc_ref.py + oracle/textblock_ref.py + oracle/pipeline_ref.py: torch
                CPU fp32 + torchvision + cv2 + numpy, i.e. the reference's own library calls) on this box's host cores.
+
+--dump-outputs DIR writes what the last timed step of `value` returned for rank 0's batch as DIR/<name>.npy (see
+step_outputs), so that two builds run with the same arguments, hence the same pages and checkpoint, can be compared
+output for output.
 """
 import argparse
 import json
@@ -157,6 +161,50 @@ def run_reference(args):
     }))
 
 
+DUMP_MASK_PIXELS = 1 << 22   # pixels kept of each batch-sized mask: 16 MB as float32 (a quarter of 16 pages of 1024^2)
+
+
+def step_outputs(arena, lay, n, h, w):
+    """The results a caller of the full-pipeline step receives for its batch of n pages (unpacked from the result
+    arena) as float32 / float64 arrays, one row per item, column 0 the page index:
+      mask_sample, mask_refined_sample  u8 masks at the same DUMP_MASK_PIXELS flat positions of the [n][h][w] batch,
+                                        np.random.default_rng(0).choice(n*h*w, DUMP_MASK_PIXELS, replace=False), sorted
+      det          page, x1, y1, x2, y2, conf, cls                  line_boxes   page, x1, y1, .. x4, y4
+      line_scores  one per line_boxes row                           n_labels / block_flags   one per page
+      blocks       page, x1, y1, x2, y2, language (LANGCLS2IDX), vertical, font_size, angle, vec x, vec y, norm,
+                   merged, weight, number of lines
+      block_lines  page, block, x1, y1, .. x4, y4
+      block_distances  page, block, distance, is_nan: a distance is NaN where the block's reading direction is degenerate
+                   (examine_textblk's arccos of 0/0, as in the reference); such rows hold distance 0 and is_nan 1 so that
+                   every value written is finite"""
+    from ctd_b200 import multigpu
+    from ctd_b200.textblock import LANGCLS2IDX
+    r = multigpu.unpack_arena(arena, lay, n, h, w, full=True)
+    px = np.sort(np.random.default_rng(0).choice(n * h * w, min(DUMP_MASK_PIXELS, n * h * w), replace=False))
+
+    def per_page(arrays, width, dtype):
+        return np.concatenate([np.concatenate([np.full((len(a), 1), i), np.reshape(a, (len(a), width - 1))], 1).astype(dtype)
+                               for i, a in enumerate(arrays)])
+
+    blocks, lines, dists = [], [], []
+    for i, page in enumerate(r["blocks"]):
+        for j, b in enumerate(page):
+            blocks.append([i, *b.xyxy, LANGCLS2IDX[b.language], b.vertical, b.font_size, b.angle, *b.vec, b.norm, b.merged,
+                           b.weight, len(b.lines)])
+            lines += [[i, j, *np.ravel(q)] for q in b.lines]
+            dists += [[i, j, 0.0, 1.0] if np.isnan(d) else [i, j, d, 0.0] for d in np.ravel(b.distance)]
+    return {"mask_sample": r["mask"].reshape(-1)[px].astype(np.float32),
+            "mask_refined_sample": r["mask_refined"].reshape(-1)[px].astype(np.float32),
+            "det": per_page(r["det"], 7, np.float32),
+            "line_boxes": per_page(r["line_boxes"], 9, np.float32),
+            "line_scores": np.concatenate(r["line_scores"]).astype(np.float32),
+            "n_labels": r["n_labels"].astype(np.float64),
+            "block_flags": np.array(r["block_flags"], np.float64),
+            "blocks": np.array(blocks, np.float64).reshape(-1, 15),
+            "block_lines": np.array(lines, np.float64).reshape(-1, 10),
+            "block_distances": np.array(dists, np.float64).reshape(-1, 4)}
+
+
 class _DevArr:
     def __init__(self, ptr, nbytes):
         self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (ptr, False), "version": 3}
@@ -178,7 +226,11 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=16,
                     help="torch intra-op threads of the CPU arm (measured on the B200 host: 16 threads 0.25 s/forward, "
                          "64 threads 0.48 s, 128 threads 33 s -- more threads only hurt)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed for rank 0's pages as DIR/<name>.npy (see step_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -306,6 +358,10 @@ def main():
         sampler.start()
     ms = timed(step_full, args.steps, drain_full)
     clocks = sampler.stop() if sampler else None
+    dump = None
+    if args.dump_outputs and rank == 0:
+        k = state["k"] - 1   # the last timed step; its host arena is reused by the steps below
+        dump = step_outputs(out_arena[k % n_eng][(k // n_eng) & 1].numpy(), lay, B, H, W)
     state["on_device"] = False
     for _ in range(2 * n_eng):
         step_full()
@@ -449,6 +505,10 @@ def main():
             line["cpu_baseline"] = {"value": ncpu / dt, "unit": "pages/s", "cores": cores, "kind": "port",
                                     "sample": "%d structured synthetic 1024x1024 pages; %s" % (ncpu, CPU_WORKLOAD)}
         print(json.dumps(line))
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     for e in engs:
         e.close()
     if dist is not None:

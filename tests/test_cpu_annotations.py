@@ -1,7 +1,11 @@
-"""not-gpu: the annotation writer (comic-text-detector_b200/annotations.py, SURVEY 8f row f2) against the UNMODIFIED
-reference's own writer code path (`model2annotations`' per-page body, inference.py:33-70, run with the reference's
-TextBlock / xyxy2yolo / get_yololabel_strings / NumpyEncoder / imwrite) on identical grouping results: every file
-byte-identical.  Needs /root/reference (build container); the format itself is also checked stand-alone."""
+"""not-gpu: the annotation writer (comic-text-detector_b200/annotations.py, SURVEY 8f row f2) against the files the
+UNMODIFIED reference's own writer code path (`model2annotations`' per-page body, inference.py:33-70, run with the
+reference's group_output / TextBlock / xyxy2yolo / get_yololabel_strings / NumpyEncoder / imwrite) wrote for the same
+pages: every file byte-identical.  What the reference wrote is stored in tests/golden/ref_annotations.json.gz (text
+files verbatim, JSON parsed, images as SHA-1 of the bytes), written by `python tests/test_cpu_annotations.py --regen`
+through oracle/ref_shim.py; the format itself is also checked stand-alone."""
+import gzip
+import hashlib
 import json
 import os
 import os.path as osp
@@ -11,12 +15,35 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ctd_b200 import annotations as ann  # noqa: E402
 from ctd_b200 import textblock as tb  # noqa: E402
 from oracle import ref_shim  # noqa: E402
 from test_cpu_textblock import make_case  # noqa: E402
 
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present on this box")
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_annotations.json.gz")
+SEEDS = [0, 3, 5, 11, 17]
+
+
+def _page(seed):
+    blks, lines, w, h, mask = make_case(seed)
+    img = np.random.default_rng(seed).integers(0, 256, (h, w, 3), dtype=np.uint8)
+    return "page %d.jpg" % seed, img, mask, (blks, lines, w, h, mask)
+
+
+def _group(fn, case):
+    blks, lines, w, h, mask = case
+    return fn((blks[0].copy(), blks[1].copy(), blks[2].copy()), lines.copy() if len(lines) else [], w, h, mask.copy())
+
+
+def _file_record(path):
+    """what the comparison keeps of a written file: text files verbatim, JSON parsed, images as SHA-1 of the bytes"""
+    data = open(path, "rb").read()
+    if path.endswith(".json"):
+        return json.loads(data)
+    if path.endswith(".txt"):
+        return data.decode("utf8")
+    return hashlib.sha1(data).hexdigest()
 
 
 def _reference_page_writer(ns, save_dir, imgname, img, mask_refined, blk_list, save_json):
@@ -44,27 +71,18 @@ def _reference_page_writer(ns, save_dir, imgname, img, mask_refined, blk_list, s
     io_utils.imwrite(osp.join(save_dir, 'mask-' + imname + '.png'), mask_refined)
 
 
-@needs_ref
-@pytest.mark.parametrize("seed", [0, 3, 5, 11, 17])
+@pytest.mark.parametrize("seed", SEEDS)
 def test_files_equal_reference_writer(tmp_path, seed):
-    ns = ref_shim.load()
-    blks, lines, w, h, mask = make_case(seed)
-    rng = np.random.default_rng(seed)
-    img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-    ours = tb.group_output((blks[0].copy(), blks[1].copy(), blks[2].copy()), lines.copy() if len(lines) else [], w, h, mask.copy())
-    theirs = ns.textblock.group_output((blks[0].copy(), blks[1].copy(), blks[2].copy()), lines.copy() if len(lines) else [], w, h, mask.copy())
-    da, db = tmp_path / "ours", tmp_path / "ref"
-    da.mkdir(); db.mkdir()
-    name = "page %d.jpg" % seed
-    ann.write_annotations(str(da), name, img, mask, ours, save_json=True)
-    _reference_page_writer(ns, str(db), name, img, mask, theirs, True)
-    fa, fb = sorted(os.listdir(da)), sorted(os.listdir(db))
-    assert fa == fb and len(fa) >= 4
+    with gzip.open(REF, "rt") as f:
+        ref = json.load(f)[str(seed)]
+    name, img, mask, case = _page(seed)
+    ann.write_annotations(str(tmp_path), name, img, mask, _group(tb.group_output, case), save_json=True)
+    fa = sorted(os.listdir(tmp_path))
+    assert fa == sorted(ref) and len(fa) >= 4
     for f in fa:
-        a, b = (da / f).read_bytes(), (db / f).read_bytes()
+        ja, jb = _file_record(str(tmp_path / f)), ref[f]
         if f.endswith(".json"):
             # same blocks, same keys, same values (key ORDER follows each class's attribute order)
-            ja, jb = json.loads(a), json.loads(b)
             assert len(ja) == len(jb)
             for x, y in zip(ja, jb):
                 for k in y:
@@ -78,7 +96,7 @@ def test_files_equal_reference_writer(tmp_path, seed):
                     else:
                         assert x[k] == y[k], (f, k)
         else:
-            assert a == b, f
+            assert ja == jb, f
 
 
 def test_label_and_line_formats(tmp_path):
@@ -92,3 +110,18 @@ def test_label_and_line_formats(tmp_path):
     ann.write_annotations(str(tmp_path), "q.jpg", img, np.zeros((400, 200), np.uint8), [], save_json=False)
     assert (tmp_path / "q.txt").read_text() == "" and not (tmp_path / "line-q.txt").exists()
     assert ann.find_all_imgs(str(tmp_path)) and all(f.endswith(".png") for f in ann.find_all_imgs(str(tmp_path)))
+
+
+if __name__ == "__main__":
+    if "--regen" in sys.argv:
+        import tempfile
+        ns = ref_shim.load()
+        rec = {}
+        for seed in SEEDS:
+            name, img, mask, case = _page(seed)
+            with tempfile.TemporaryDirectory() as d:
+                _reference_page_writer(ns, d, name, img, mask, _group(ns.textblock.group_output, case), True)
+                rec[str(seed)] = {f: _file_record(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+        with open(REF, "wb") as f:
+            f.write(gzip.compress(json.dumps(rec, sort_keys=True).encode(), 9, mtime=0))
+        print("wrote", REF)

@@ -1,45 +1,46 @@
-"""not-gpu: pin the oracle.  (a) against the UNMODIFIED reference when /root/reference is present
-(build container), (b) always against the committed golden vectors the reference produced
-(tests/golden/, generated by oracle/make_golden.py)."""
+"""not-gpu: pin the oracle against what the UNMODIFIED reference computed on the same inputs: the committed golden
+vectors under tests/golden/ (net_*_256.npz and nms_ref.npz from oracle/make_golden.py, ref_*.npz from
+`python tests/test_cpu_oracle.py --regen`; both import the reference through oracle/ref_shim.py)."""
 import os
 
 import numpy as np
 import pytest
 import sys
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 
 from oracle import geom_ref, postproc_ref, ref_shim, synth
 from oracle.net_ref import RefNet
-from util import page_to_net_input
+from util import page_to_net_input, reference_threads
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present on this box")
+REF_NET = os.path.join(GOLD, "ref_net_rough_128x192.npz")
+REF_SEG = os.path.join(GOLD, "ref_seg_represent.npz")
 
 
-@needs_ref
-def test_net_ref_is_bit_identical_to_reference(tmp_path):
-    ns = ref_shim.load()
+def _net_case():
+    """rough checkpoint (every tap random) on one 128x192 page"""
     ck = synth.make_checkpoint(0, smooth=False, bn_calibrate=128)
-    f = str(tmp_path / "ck.pt")
-    torch.save(ck, f)
-    net = ns.basemodel.TextDetBase(f, device="cpu", act="leaky")
-    pages = np.stack([synth.structured_page(3, 128, 192)])
-    x = page_to_net_input(pages)
-    with torch.no_grad():
-        rb, rm, rl = net(x)
-    b, m, l = RefNet(ck)(x)
-    assert torch.equal(b, rb) and torch.equal(m, rm) and torch.equal(l, rl)
+    return ck, page_to_net_input(np.stack([synth.structured_page(3, 128, 192)]))
 
 
-@needs_ref
+def test_net_ref_is_bit_identical_to_reference():
+    """RefNet == the reference's TextDetBase forward (stored), bit for bit"""
+    g = np.load(REF_NET)
+    with reference_threads():
+        ck, x = _net_case()
+        b, m, l = RefNet(ck)(x)
+    assert torch.equal(b, torch.from_numpy(g["blks"])) and torch.equal(m, torch.from_numpy(g["mask"])) and \
+        torch.equal(l, torch.from_numpy(g["lines"]))
+
+
 def test_nms_restatement_equals_reference():
-    ns = ref_shim.load()
+    """nms_ref.npz holds the reference's non_max_suppression output for its `pred`"""
     g = np.load(os.path.join(GOLD, "nms_ref.npz"))
     pred = torch.from_numpy(g["pred"])[None]
-    ref = ns.yolov5_utils.non_max_suppression(pred.clone(), 0.4, 0.35)[0]
     got = postproc_ref.non_max_suppression(pred, 0.4, 0.35)[0]
-    assert torch.equal(ref, got)
+    assert torch.equal(torch.from_numpy(g["det"]), got)
 
 
 @pytest.mark.parametrize("name", ["net_smooth_256.npz", "net_rough_256.npz"])
@@ -80,15 +81,39 @@ def test_geos_restatements():
     assert geom_ref.polygons_intersect(sq, [(1, 1), (2, 1), (2, 2), (1, 2)])       # containment
 
 
-@needs_ref
 def test_seg_represent_restatement_equals_reference_class():
-    """oracle/postproc_ref.seg_represent == the reference's SegDetectorRepresenter (pyclipper/shapely shimmed
-    by oracle/geom_ref.py on BOTH sides, hence 'parity unpinned' for those two calls only)."""
+    """oracle/postproc_ref.seg_represent == the reference's SegDetectorRepresenter (stored; pyclipper/shapely were
+    shimmed by oracle/geom_ref.py when it ran, hence 'parity unpinned' for those two calls only)."""
+    import stress_maps
+    g = np.load(REF_SEG)
+    assert sorted(g.files) == sorted(k + "_" + name for name in stress_maps.CASES for k in ("boxes", "scores"))
+    for name, f in stress_maps.CASES.items():
+        ob, os_ = postproc_ref.seg_represent(f(), 0.3)
+        assert np.array_equal(g["boxes_" + name], ob) and np.array_equal(g["scores_" + name], os_), name
+
+
+def regen():
+    """Runs the unmodified reference (oracle/ref_shim.py) and writes the ref_*.npz vectors the tests above read."""
+    import tempfile
     import stress_maps
     ns = ref_shim.load()
+    with reference_threads(), tempfile.TemporaryDirectory() as d:
+        ck, x = _net_case()
+        f = os.path.join(d, "ck.pt")
+        torch.save(ck, f)
+        net = ns.basemodel.TextDetBase(f, device="cpu", act="leaky")
+        with torch.no_grad():
+            rb, rm, rl = net(x)
+    np.savez_compressed(REF_NET, blks=rb.numpy(), mask=rm.numpy(), lines=rl.numpy())
     rep = ns.db_utils.SegDetectorRepresenter(thresh=0.3)
-    for name, f in stress_maps.CASES.items():
-        pred = f()
-        b, s = rep(None, torch.from_numpy(pred)[None, None])
-        ob, os_ = postproc_ref.seg_represent(pred, 0.3)
-        assert np.array_equal(b[0], ob) and np.array_equal(s[0], os_), name
+    seg = {}
+    for name, fn in stress_maps.CASES.items():
+        b, s = rep(None, torch.from_numpy(fn())[None, None])
+        seg["boxes_" + name], seg["scores_" + name] = np.asarray(b[0]), np.asarray(s[0])
+    np.savez_compressed(REF_SEG, **seg)
+    print("wrote", REF_NET, REF_SEG)
+
+
+if __name__ == "__main__":
+    if "--regen" in sys.argv:
+        regen()

@@ -1,8 +1,8 @@
-"""not-gpu: the remaining oracle pins (VERDICT r1 #6).  In the build container (/root/reference present) the oracle's
-`refine_mask`, `refine_undetected_mask` and the whole post-network chain are compared with the UNMODIFIED reference
-(`utils.textmask.refine_mask`, `utils.textmask.refine_undetected_mask`, `inference.TextDetector.__call__`); everywhere
-they are compared with golden digests the reference produced (tests/golden/pins.json, written by
-`python tests/test_cpu_oracle_pins.py --regen` in the build container).
+"""not-gpu: the remaining oracle pins (VERDICT r1 #6).  The oracle's `refine_mask`, `refine_undetected_mask` and the
+whole post-network chain are compared with what the UNMODIFIED reference (`utils.textmask.refine_mask`,
+`utils.textmask.refine_undetected_mask`, `inference.TextDetector.__call__`) returned for the same inputs
+(tests/golden/ref_postprocess.npz) and with golden digests checked against the reference (tests/golden/pins.json); both
+are written by `python tests/test_cpu_oracle_pins.py --regen`, which imports the reference through oracle/ref_shim.py.
 
 One documented normalisation (SURVEY 8c): `get_topk_color` sorts the histogram with `np.argsort(bins * -1)`, an UNSTABLE
 sort whose tie order depends on numpy's SIMD build; the oracle (and the CUDA kernel) break ties by ascending bin index.
@@ -19,9 +19,10 @@ import pytest
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import pipeline_ref, postproc_ref, ref_shim, synth, textblock_ref  # noqa: E402
+from util import reference_threads  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pins.json")
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present on this box")
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_postprocess.npz")
 
 
 def _digest(a):
@@ -54,62 +55,61 @@ class _Blk:
         self.xyxy = xyxy
 
 
-@needs_ref
+def _reference():
+    return np.load(REF)
+
+
 @pytest.mark.parametrize("mode", [0, 1])
 @pytest.mark.parametrize("seed", range(8))
 def test_refine_mask_equals_reference(seed, mode):
-    ns = ref_shim.load()
     img, mask, boxes = refine_case(seed)
-    ref = ns.textmask.refine_mask(img, mask.copy(), [_Blk(b) for b in boxes], refine_mode=mode)
     got = postproc_ref.refine_mask(img, mask.copy(), boxes, mode, tie_order="numpy")
-    assert np.array_equal(ref, got)
+    assert np.array_equal(_reference()["refine_%d_%d" % (seed, mode)], got)
 
 
-@needs_ref
+def _undetected_case(seed):
+    img, mask, boxes = refine_case(20 + seed)
+    return img, mask, boxes[: max(1, len(boxes) // 2)]          # the other blobs are "undetected"
+
+
 @pytest.mark.parametrize("seed", range(6))
 def test_refine_undetected_mask_equals_reference(seed):
-    ns = ref_shim.load()
-    img, mask, boxes = refine_case(20 + seed)
-    kept = boxes[: max(1, len(boxes) // 2)]          # the other blobs are "undetected"
-    refined = ns.textmask.refine_mask(img, mask.copy(), [_Blk(b) for b in kept], refine_mode=0)
-    m_ref, m_got = mask.copy(), mask.copy()
-    ref = ns.textmask.refine_undetected_mask(img, m_ref, refined.copy(), [_Blk(b) for b in kept], refine_mode=0)
+    img, mask, kept = _undetected_case(seed)
+    g = _reference()
+    refined = g["undetected_refined_%d" % seed]     # the reference's refine_mask of the kept blocks
+    m_got = mask.copy()
     got = pipeline_ref.refine_undetected_mask(img, m_got, refined.copy(), kept, None, 0, tie_order="numpy")
-    assert np.array_equal(ref, got) and np.array_equal(m_ref, m_got)     # incl. the in-place edit of mask_pred
+    # incl. the in-place edit of mask_pred
+    assert np.array_equal(g["undetected_%d" % seed], got) and np.array_equal(g["undetected_mask_%d" % seed], m_got)
 
 
 def _chain_case(seed, size=256):
     import torch
     from oracle.net_ref import RefNet
-    ck = synth.make_checkpoint(0, smooth=True)
     page = synth.structured_page(1000 + seed, size, size)
     x = torch.from_numpy(np.ascontiguousarray(page.transpose(2, 0, 1))[None].astype(np.float32) / 255)
-    with torch.no_grad():
+    with reference_threads(), torch.no_grad():
+        ck = synth.make_checkpoint(0, smooth=True)
         blks, mask, lines = RefNet(ck)(x)
     return ck, page, blks[0].numpy(), mask[0, 0].numpy(), lines[0].numpy()
 
 
-@needs_ref
+def _block_keys(blk_list):
+    return [[[int(v) for v in x.xyxy], np.array(x.lines).tolist(), x.language, bool(x.vertical)] for x in blk_list]
+
+
 @pytest.mark.parametrize("keep", [False, True])
 @pytest.mark.parametrize("seed", [0, 3])
-def test_full_chain_equals_unmodified_text_detector(tmp_path, seed, keep):
-    """inference.TextDetector.__call__ (reference, CPU torch backend) vs RefNet + oracle chain on the same page."""
-    import torch
-    ns = ref_shim.load()
-    ck, page, blks, mask, lines = _chain_case(seed)
-    f = str(tmp_path / "ck.pt")
-    torch.save(ck, f)
-    det = ns.inference.TextDetector(f, input_size=256, device="cpu", act="leaky")
-    m_ref, r_ref, b_ref = det(page.copy(), keep_undetected_mask=keep)
-    m, r, b = pipeline_ref.postprocess_page(page.copy(), blks, mask, lines, ns.textblock.group_output, keep_undetected_mask=keep,
+def test_full_chain_equals_unmodified_text_detector(seed, keep):
+    """inference.TextDetector.__call__ (reference, CPU torch backend, stored) vs RefNet + oracle chain (with the oracle's
+    python group_output restatement) on the same page."""
+    _ck, page, blks, mask, lines = _chain_case(seed)
+    g = _reference()
+    m, r, b = pipeline_ref.postprocess_page(page.copy(), blks, mask, lines, textblock_ref.group_output, keep_undetected_mask=keep,
                                             tie_order="numpy")
-    assert np.array_equal(m, m_ref) and np.array_equal(r, r_ref)
-    assert [(x.xyxy, np.array(x.lines).tolist(), x.language, bool(x.vertical)) for x in b] == \
-        [(x.xyxy, np.array(x.lines).tolist(), x.language, bool(x.vertical)) for x in b_ref]
-    # and with the oracle's own (python) group_output restatement
-    m2, r2, b2 = pipeline_ref.postprocess_page(page.copy(), blks, mask, lines, textblock_ref.group_output, keep_undetected_mask=keep,
-                                               tie_order="numpy")
-    assert np.array_equal(r2, r_ref) and len(b2) == len(b_ref)
+    tag = "%d_%d" % (seed, keep)
+    assert _digest(m) == str(g["chain_mask_" + tag]) and np.array_equal(r, g["chain_refined_" + tag])
+    assert _block_keys(b) == json.loads(str(g["chain_blocks_" + tag]))
 
 
 def _golden_records():
@@ -161,10 +161,43 @@ def test_argsort_tie_pixels_are_counted():
     print("pixels changed by the stable-tie normalisation per case:", now)
 
 
+def _reference_records(ns):
+    """what the unmodified reference returns for every case the *_equals_reference / *_unmodified_* tests compare"""
+    import tempfile
+    import torch
+    rec = {}
+    for mode in (0, 1):
+        for seed in range(8):
+            img, mask, boxes = refine_case(seed)
+            rec["refine_%d_%d" % (seed, mode)] = ns.textmask.refine_mask(img, mask.copy(), [_Blk(b) for b in boxes], refine_mode=mode)
+    for seed in range(6):
+        img, mask, kept = _undetected_case(seed)
+        refined = ns.textmask.refine_mask(img, mask.copy(), [_Blk(b) for b in kept], refine_mode=0)
+        m_ref = mask.copy()
+        rec["undetected_refined_%d" % seed] = refined.copy()
+        rec["undetected_%d" % seed] = ns.textmask.refine_undetected_mask(img, m_ref, refined, [_Blk(b) for b in kept], refine_mode=0)
+        rec["undetected_mask_%d" % seed] = m_ref
+    for seed in (0, 3):
+        ck, page, _blks, _mask, _lines = _chain_case(seed)
+        with tempfile.TemporaryDirectory() as d:
+            f = os.path.join(d, "ck.pt")
+            torch.save(ck, f)
+            det = ns.inference.TextDetector(f, input_size=256, device="cpu", act="leaky")
+        for keep in (False, True):
+            m_ref, r_ref, b_ref = det(page.copy(), keep_undetected_mask=keep)
+            tag = "%d_%d" % (seed, keep)
+            # the grey-level mask as a digest: it is the bulk of the file and the network test pins the map behind it
+            rec["chain_mask_" + tag], rec["chain_refined_" + tag] = np.array(_digest(m_ref)), r_ref
+            rec["chain_blocks_" + tag] = np.array(json.dumps(_block_keys(b_ref)))
+    return rec
+
+
 if __name__ == "__main__":
     if "--regen" in sys.argv:
-        assert ref_shim.available(), "regenerate in the build container (needs /root/reference)"
         ns = ref_shim.load()
+        with reference_threads():
+            np.savez_compressed(REF, **_reference_records(ns))
+        print("wrote", REF)
         # every digest written here is first checked against the unmodified reference
         for mode in (0, 1):
             for seed in range(8):

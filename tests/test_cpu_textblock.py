@@ -1,9 +1,12 @@
 """not-gpu: the native line -> block grouping (`ctd_group_output`, csrc/group.cpp, called through
-comic-text-detector_b200/textblock.py) AND the oracle's python restatement (oracle/textblock_ref.py) against the
-unmodified reference `utils.textblock.group_output` on identical random inputs (build container), and against golden
-results the reference produced (tests/golden/group_output.json, everywhere).  Integer fields, structure and order must
-be identical; float fields are compared to 1e-12 relative for the native code (glibc acos/sin vs numpy's SIMD
-kernels may differ in the last ulp) and exactly for the python restatement."""
+comic-text-detector_b200/textblock.py) AND the oracle's python restatement (oracle/textblock_ref.py) against what the
+unmodified reference `utils.textblock.group_output` returned on identical random inputs (tests/golden/group_output.json
+and tests/golden/ref_group_output.json.gz, the latter written by `python tests/test_cpu_textblock.py --regen` through
+oracle/ref_shim.py).  Integer fields, structure and order must be identical; float fields are compared to 1e-12
+relative for the native code (glibc acos/sin vs numpy's SIMD kernels may differ in the last ulp) and exactly for the
+python restatement."""
+import functools
+import gzip
 import json
 import os
 import sys
@@ -12,11 +15,12 @@ import numpy as np
 import pytest
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ctd_b200 import textblock as tb  # noqa: E402
 from oracle import ref_shim, textblock_ref  # noqa: E402
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "group_output.json")
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present on this box")
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_group_output.json.gz")
 
 
 def make_case(seed, im_w=1024, im_h=1024):
@@ -84,20 +88,25 @@ def assert_same_blocks(got, ref, rel=1e-12):
                 assert g[k] == r[k], (i, k, g[k], r[k])
 
 
-@needs_ref
+def reference_case(seed):
+    return make_case(seed) if seed < 48 else make_case(seed, 1536, 1024)     # landscape pages halve the grid width
+
+
+@functools.lru_cache(maxsize=None)
+def reference_blocks():
+    """seed -> blk_summary list of the reference's group_output on reference_case(seed), seeds 0..63"""
+    with gzip.open(REF, "rt") as f:
+        return json.load(f)
+
+
 @pytest.mark.parametrize("seed", range(24))
 def test_python_restatement_equals_reference(seed):
-    ns = ref_shim.load()
-    case = make_case(seed)
-    assert _run(textblock_ref.group_output, case) == _run(ns.textblock.group_output, case)
+    assert _run(textblock_ref.group_output, make_case(seed)) == reference_blocks()[str(seed)]
 
 
-@needs_ref
 @pytest.mark.parametrize("seed", range(64))
 def test_native_group_output_equals_reference(seed):
-    ns = ref_shim.load()
-    case = make_case(seed) if seed < 48 else make_case(seed, 1536, 1024)     # landscape pages halve the grid width
-    assert_same_blocks(_run(tb.group_output, case), _run(ns.textblock.group_output, case))
+    assert_same_blocks(_run(tb.group_output, reference_case(seed)), reference_blocks()[str(seed)])
 
 
 def test_native_group_output_golden():
@@ -137,3 +146,12 @@ def test_quads_intersect():
     assert textblock_ref.quads_intersect(sq, [(4, 3), (6, 3), (6, 5), (4, 5)])
     assert not textblock_ref.quads_intersect(sq, [(5, 0), (6, 0), (6, 1), (5, 1)])
     assert textblock_ref.quads_intersect(sq, [(1, 1), (2, 1), (2, 2), (1, 2)])
+
+
+if __name__ == "__main__":
+    if "--regen" in sys.argv:
+        ns = ref_shim.load()
+        rec = {str(seed): _run(ns.textblock.group_output, reference_case(seed)) for seed in range(64)}
+        with open(REF, "wb") as f:
+            f.write(gzip.compress(json.dumps(rec, sort_keys=True).encode(), 9, mtime=0))
+        print("wrote", REF)

@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests."""
+import contextlib
 import os
 import sys
 
@@ -14,6 +15,20 @@ from ctd_b200 import compiler as cc  # noqa: E402
 from ctd_b200.binding import PREC_FP16_TC, PREC_FP32_SIMT, PREC_FP16_SIMT, PREC_SPLIT_TC  # noqa: E402
 
 _CKPT_CACHE = {}
+
+REFERENCE_THREADS = 8   # torch CPU threads the stored reference outputs (tests/golden/ref_*) were computed with
+
+
+@contextlib.contextmanager
+def reference_threads():
+    """torch's CPU kernels split their sums by thread count and each split rounds differently, so a float result (the
+    BN statistics of a synthetic checkpoint, a network map) is reproduced bit for bit only with the same count."""
+    old = torch.get_num_threads()
+    torch.set_num_threads(REFERENCE_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(old)
 
 
 def get_checkpoint(seed=0, smooth=True):

@@ -1,8 +1,10 @@
 """Per-op device time of the forward with the yolo activations as compiled (SiLU) vs replaced by LeakyReLU (no MUFU):
 how much of each layer's time is the SiLU epilogue.  (Experiment only: the LeakyReLU program is not a valid model.)"""
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from ctd_b200 import compiler as cc
 from oracle import synth

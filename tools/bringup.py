@@ -1,8 +1,9 @@
 """GPU bring-up diagnostics (not a test): per-stage error report + timings.  Run under gpurun."""
-import sys, time
+import os, sys, time
 import numpy as np
 import torch
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from ctd_b200.binding import PREC_FP16_TC, PREC_FP32_SIMT, PREC_FP16_SIMT
 from oracle import synth

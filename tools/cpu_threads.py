@@ -1,6 +1,7 @@
 """How does the reference's CPU forward scale with torch threads on this host? (for bench.py --cpu-threads)"""
-import sys, time
-sys.path.insert(0, "/root/repo")
+import os, sys, time
+ROOT =os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import numpy as np, torch
 from oracle import synth
 from oracle.net_ref import RefNet

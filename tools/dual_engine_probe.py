@@ -1,11 +1,13 @@
 """Probe: does running two engines (two CUDA graphs on two streams) back to back raise whole-GPU throughput?"""
+import os
 import sys
 import time
 
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from oracle import synth
 

@@ -1,11 +1,13 @@
 """Net-level error of each engine precision against the fp32 oracle at several page sizes (GPU box)."""
+import os
 import sys
 
 import numpy as np
 import torch
 
-sys.path.insert(0, "/root/repo")
-sys.path.insert(0, "/root/repo/tests")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ctd_b200
 from oracle import synth
 from oracle.net_ref import RefNet

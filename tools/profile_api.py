@@ -1,12 +1,14 @@
 """cProfile of the drop-in TextDetector.__call__ on synthetic pages (where does the per-page host time go)."""
 import cProfile
 import pstats
+import os
 import sys
 import time
 
 import numpy as np
 
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from oracle import synth
 

@@ -1,7 +1,9 @@
 """Runs a few forwards of the synthetic checkpoint (for ncu launch lists / captures)."""
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from oracle import synth
 

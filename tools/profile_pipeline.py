@@ -1,9 +1,11 @@
 """Runs a few FULL-pipeline batches (ctd_submit_full / ctd_collect: network + post-processing + group_output +
 refine_mask) of the synthetic checkpoint, one batch at a time (for ncu launch lists / captures)."""
+import os
 import sys
 import numpy as np
 import torch
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from oracle import synth
 

@@ -1,7 +1,9 @@
 """refine_mask of ONE synthetic page's windows, twice (for ncu captures of refine_kernel)."""
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from ctd_b200.inference import expand_textwindow
 from oracle import synth

@@ -1,11 +1,13 @@
 """How long does refine_mask take on the synthetic 1024x1024 pages, and how are the window sizes distributed?
 (sizing input for the batched device pipeline; run on the GPU box)"""
+import os
 import sys
 import time
 
 import numpy as np
 
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import ctd_b200
 from ctd_b200.inference import expand_textwindow
 from oracle import synth

@@ -7,9 +7,10 @@ OUT=gpurun_out
 mkdir -p $OUT
 CS="compute-sanitizer --print-limit 5 --launch-timeout 120"
 cat > /tmp/fullpipe_small.py <<'PY'
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+sys.path.insert(0, os.getcwd()); sys.path.insert(0, os.path.join(os.getcwd(), "tests"))
 import ctd_b200
 from oracle import synth
 from util import get_checkpoint

@@ -9,9 +9,10 @@ CS="compute-sanitizer --print-limit 5 --launch-timeout 120"
 timeout 900 $CS --tool memcheck python -m pytest tests/test_gpu_kernels.py -q -m gpu -x 2>&1 | tail -25 > $OUT/sanitizer_memcheck_kernels.log
 timeout 600 $CS --tool memcheck python -m pytest tests/test_gpu_refine.py -q -m gpu -x 2>&1 | tail -25 > $OUT/sanitizer_memcheck_refine.log
 cat > /tmp/fullpipe_small.py <<'PY'
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+sys.path.insert(0, os.getcwd()); sys.path.insert(0, os.path.join(os.getcwd(), "tests"))
 import ctd_b200
 from oracle import synth
 from util import get_checkpoint

@@ -1,7 +1,9 @@
 """tiny split-fp16 forward (for compute-sanitizer runs)"""
+import os
 import sys
 import numpy as np
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ctd_b200
 from oracle import synth
 from util import get_checkpoint
