@@ -54,6 +54,13 @@ class CtdResultsLayout(C.Structure):
 
 MAX_BLOCKS, MAX_BLOCK_DIST = 1300, 8192   # CTD_MAX_BLOCKS / CTD_MAX_BLOCK_DIST
 
+# numpy mirror of `ctd_region` (include/ctd_b200.h) and its flag / status values
+REGION_DTYPE = np.dtype([("status", np.int32), ("out_h", np.int32), ("out_w", np.int32), ("w", np.int32),
+                         ("h", np.int32), ("reserved", np.int32), ("offset", np.uint64), ("bytes", np.uint64),
+                         ("M", np.float64, (9,))], align=True)
+REGION_EXPAND, REGION_VERTICAL = 1, 2
+REGION_OK, REGION_E_RATIO, REGION_E_HOMOGRAPHY, REGION_E_SIZE = 0, 1, 2, 3
+
 EXPORTS = ["ctd_create", "ctd_destroy", "ctd_last_error", "ctd_forward", "ctd_get_net_outputs", "ctd_get_mask_u8",
            "ctd_get_detections", "ctd_get_db_components", "ctd_last_forward_ms", "ctd_last_launch_count",
            "ctd_debug_read_buffer", "ctd_debug_write_buffer", "ctd_connected_components", "ctd_nms",
@@ -61,7 +68,8 @@ EXPORTS = ["ctd_create", "ctd_destroy", "ctd_last_error", "ctd_forward", "ctd_ge
            "ctd_get_text_lines", "ctd_seg_represent", "ctd_refine_mask", "ctd_submit", "ctd_collect",
            "ctd_results_bytes", "ctd_join", "ctd_forward_resized", "ctd_get_mask_u8_resized",
            "ctd_resize_linear_u8", "ctd_debug_run_ops", "ctd_get_nms_status", "ctd_group_output",
-           "ctd_expand_textwindow", "ctd_detect_page", "ctd_results_layout", "ctd_submit_full", "ctd_device_arena"]
+           "ctd_expand_textwindow", "ctd_detect_page", "ctd_results_layout", "ctd_submit_full", "ctd_device_arena",
+           "ctd_plan_regions", "ctd_transform_regions"]
 
 _lib = None
 
@@ -119,6 +127,9 @@ def load_library():
     lib.ctd_results_layout.argtypes = [vp, C.POINTER(CtdResultsLayout)]
     lib.ctd_submit_full.argtypes = [vp, i32, vp, i32, i32, i32, i32, i32, vp]
     lib.ctd_device_arena.argtypes = [vp, i32, C.POINTER(vp), C.POINTER(vp)]
+    lib.ctd_plan_regions.argtypes = [vp, vp, vp, i32, i32, i32, i32, C.c_double, vp, C.POINTER(C.c_size_t)]
+    lib.ctd_transform_regions.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, vp, i32, C.c_double, vp, vp, i32,
+                                          C.c_size_t]
     for name in EXPORTS[3:]:
         getattr(lib, name).restype = C.c_int
     lib.ctd_expand_textwindow.restype = None
@@ -128,6 +139,28 @@ def load_library():
 
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _region_args(quads, flags, font_size):
+    quads = np.ascontiguousarray(np.asarray(quads, np.float64).reshape(-1, 4, 2))
+    flags = np.ascontiguousarray(np.asarray(flags, np.int32).reshape(-1))
+    font_size = np.ascontiguousarray(np.asarray(font_size, np.float64).reshape(-1))
+    assert len(flags) == len(quads) and len(font_size) == len(quads), (quads.shape, flags.shape, font_size.shape)
+    return quads, flags, font_size
+
+
+def plan_regions(quads, flags, font_size, im_w, im_h, channels, textheight):
+    """ctd_plan_regions (host only, no handle): per-line status / crop shape / packed offset of
+    `TextBlock.get_transformed_region` -> (REGION_DTYPE records, total bytes)."""
+    lib = load_library()
+    quads, flags, font_size = _region_args(quads, flags, font_size)
+    rec = np.zeros((len(quads),), REGION_DTYPE)
+    total = C.c_size_t()
+    rc = lib.ctd_plan_regions(_ptr(quads), _ptr(flags), _ptr(font_size), len(quads), int(im_w), int(im_h), int(channels),
+                              float(textheight), _ptr(rec), C.byref(total))
+    if rc != 0:
+        raise CtdError("ctd_plan_regions failed (%d)" % rc)
+    return rec, int(total.value)
 
 
 class Engine:
@@ -370,6 +403,34 @@ class Engine:
                                           MAX_BLOCK_DIST, C.byref(nb)))
         self.shape = (1, net_h, net_w)
         return mask, refined, rec[:nb.value], lines, dist
+
+    def transform_regions(self, img, quads, flags, font_size, textheight, out=None, img_dev=None, out_dev=None,
+                          out_bytes=None):
+        """every line crop of one page in one call (ctd_transform_regions) -> (REGION_DTYPE records, packed u8 output).
+        img: u8 [H,W] or [H,W,C] host array, or with img_dev = (device pointer, H, W, C) a page already in HBM.
+        out: host u8 array to fill (allocated from the plan when None); with out_dev = device pointer the crops stay on
+        the device (out_bytes = its capacity) and the second result is None."""
+        quads, flags, font_size = _region_args(quads, flags, font_size)
+        if img_dev is None:
+            img = np.ascontiguousarray(img, np.uint8)
+            ih, iw = img.shape[:2]
+            ch = 1 if img.ndim == 2 else img.shape[2]
+            src, on_dev = _ptr(img), 0
+        else:
+            ptr, ih, iw, ch = img_dev
+            src, on_dev = C.c_void_p(ptr), 1
+        rec = np.zeros((len(quads),), REGION_DTYPE)
+        if out_dev is not None:
+            dst, cap = C.c_void_p(out_dev), int(out_bytes)
+        else:
+            if out is None:   # other channel counts are rejected by the call itself (CTD_E_INVALID)
+                total = plan_regions(quads, flags, font_size, iw, ih, ch, textheight)[1] if ch in (1, 3) else 0
+                out = np.empty((total,), np.uint8)
+            dst, cap = _ptr(out), out.nbytes if out_bytes is None else int(out_bytes)
+        self._ck(self.lib.ctd_transform_regions(self.h, src, ih, iw, ch, on_dev, _ptr(quads), _ptr(flags), _ptr(font_size),
+                                                len(quads), float(textheight), _ptr(rec), dst, int(out_dev is not None),
+                                                cap))
+        return rec, (None if out_dev is not None else out)
 
     def collect(self, slot):
         self._ck(self.lib.ctd_collect(self.h, slot))

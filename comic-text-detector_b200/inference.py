@@ -9,17 +9,34 @@ Everything runs in libctd_b200.so: network, NMS, mask u8, DB binarize, connected
 refine_mask on the GPU; ratio scaling, `group_output` and the window expansion in host C++ (csrc/group.cpp,
 csrc/pipeline.cu).  This module is the reference-shaped Python surface over `ctd_detect_page`.
 """
+import weakref
 from pathlib import Path
 from typing import List
 
 import numpy as np
 
 from . import compiler
-from .binding import Engine, PREC_FP16_TC, PREC_FP32_SIMT
+from .binding import Engine, PREC_FP16_TC, PREC_FP32_SIMT, REGION_EXPAND, REGION_OK, REGION_VERTICAL
 from .textblock import TextBlock, blocks_from_records, group_output, overlap_area  # noqa: F401
 
 REFINEMASK_INPAINT = 0
 REFINEMASK_ANNOTATION = 1
+
+
+_LIVE_DETECTOR = None   # weak reference to the most recently created TextDetector (TextBlock.get_transformed_region)
+
+
+def live_detector():
+    """the most recently created TextDetector if it is still alive and open, else None"""
+    det = _LIVE_DETECTOR() if _LIVE_DETECTOR is not None else None
+    return det if det is not None and det.net.h else None
+
+
+# what the reference raises for a line it cannot crop, by ctd_region status (textblock.py:175-191)
+_REGION_ERRORS = {1: "the line's aspect ratio is 0, inf or nan (round() raises OverflowError / ValueError)",
+                  2: "cv2.findHomography returns None for this line (w or h is 1, or the quad has no extent along an "
+                     "axis), so cv2.warpPerspective raises cv2.error",
+                  3: "the crop would exceed 2 GiB"}
 
 
 def letterbox_geometry(shape_hw, new_shape=(1024, 1024)):
@@ -80,6 +97,8 @@ class TextDetector:
         # DB threshold is hard-coded 0.3 in the reference (inference.py:139 ignores mask_thresh)
         self.net = Engine(self.program, device=device_index, precision=precision, max_batch=1, max_h=input_size[0],
                           max_w=input_size[1], conf_thresh=conf_thresh, nms_thresh=nms_thresh, db_thresh=0.3)
+        global _LIVE_DETECTOR
+        _LIVE_DETECTOR = weakref.ref(self)
 
     def close(self):
         self.net.close()
@@ -93,3 +112,40 @@ class TextDetector:
         mask, mask_refined, rec, lines, dist = self.net.detect_page(img, self.input_size[0], self.input_size[1], refine_mode,
                                                                     keep_undetected_mask)
         return mask, mask_refined, blocks_from_records(rec, lines, dist)
+
+    def get_transformed_regions(self, img, blk_list, textheight):
+        """`TextBlock.get_transformed_region(img, idx, textheight)` (reference utils/textblock.py:162-194) for every line
+        of every block, in one native call (ctd_transform_regions: homographies and warps on the GPU, bit-exact with
+        cv2.findHomography + cv2.warpPerspective).  Returns one list per block with one uint8 crop per line in the
+        reference's shape (h x w, or w x h rotated for vertical lines; 2-D for a 2-D or single-channel page), and None
+        for a line on which the reference raises.  The crops are views of one packed buffer."""
+        items = [(blk, i) for blk in blk_list for i in range(len(blk.lines))]
+        crops, _status = self._crop_lines(img, items, textheight)
+        out, k = [], 0
+        for blk in blk_list:
+            out.append(crops[k:k + len(blk.lines)])
+            k += len(blk.lines)
+        return out
+
+    def _crop_lines(self, img, items, textheight):
+        """(blk, line index) pairs -> (list of crops or None, ctd_region statuses)"""
+        img = np.ascontiguousarray(img)
+        if img.dtype != np.uint8 or img.ndim not in (2, 3):
+            raise ValueError("expected a uint8 HxW or HxWxC page, got %s %s" % (img.dtype, img.shape))
+        ch = 1 if img.ndim == 2 else img.shape[2]
+        if not items:
+            return [], []
+        quads = np.array([np.asarray(blk.lines[i], np.float64).reshape(4, 2) for blk, i in items])
+        flags = np.array([(REGION_EXPAND if blk.language == "eng" or (blk.language == "unknown" and not blk.vertical)
+                           else 0) | (REGION_VERTICAL if blk.vertical else 0) for blk, _i in items], np.int32)
+        font = np.array([blk.font_size for blk, _i in items], np.float64)
+        rec, buf = self.net.transform_regions(img, quads, flags, font, float(textheight))
+        crops = []
+        for r in rec.tolist():
+            status, out_h, out_w, off, nbytes = r[0], r[1], r[2], r[6], r[7]
+            if status != REGION_OK:
+                crops.append(None)
+                continue
+            crop = buf[off:off + nbytes]
+            crops.append(crop.reshape(out_h, out_w) if ch == 1 else crop.reshape(out_h, out_w, ch))
+        return crops, rec["status"].tolist()

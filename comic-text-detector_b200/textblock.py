@@ -18,8 +18,10 @@ LANGCLS2IDX = {"eng": 0, "ja": 1, "unknown": 2}
 
 
 class TextBlock(object):
-    """Result record with the reference's field names (textblock.py:12-85); the UI/OCR helpers of the
-    reference class (min_rect, get_transformed_region, colours ...) are not part of the detection path."""
+    """Result record with the reference's field names (textblock.py:12-85).  `get_transformed_region` (the OCR crop
+    of one line, textblock.py:162-194) runs on the GPU through the most recently created live `TextDetector`; the
+    other UI helpers of the reference class (min_rect, colours ...) are not part of the detection path.  Instances
+    carry only the reference's attributes: `vars(blk)` feeds to_dict and the annotation writer."""
 
     def __init__(self, xyxy, lines=None, language="unknown", vertical=False, font_size=-1, distance=None, angle=0,
                  vec=None, norm=-1, merged=False, weight=-1, text=None, translation="", fg_r=0, fg_g=0, fg_b=0,
@@ -64,6 +66,21 @@ class TextBlock(object):
 
     def to_dict(self):
         return copy.deepcopy(vars(self))
+
+    def get_transformed_region(self, img, idx, textheight):
+        """reference textblock.py:162-194: line `idx` cropped from the page and straightened to `textheight` pixels
+        (rotated 90 degrees counter-clockwise for vertical blocks), bit-exact with the reference's cv2 calls.  Runs on the
+        GPU of the most recently created live TextDetector (RuntimeError when there is none; there is no CPU path);
+        raises ValueError where the reference raises (OverflowError / ValueError / cv2.error)."""
+        from .inference import live_detector, _REGION_ERRORS
+        det = live_detector()
+        if det is None:
+            raise RuntimeError("TextBlock.get_transformed_region runs on a TextDetector's GPU engine; create one first")
+        self.lines[idx]   # IndexError like the reference
+        crops, status = det._crop_lines(img, [(self, idx)], textheight)
+        if crops[0] is None:
+            raise ValueError("line %d cannot be cropped: %s" % (idx, _REGION_ERRORS.get(status[0], status[0])))
+        return crops[0]
 
 
 def blocks_from_records(blocks, lines, dist):

@@ -363,6 +363,46 @@ CTD_API int ctd_submit_full(ctd_handle* h, int32_t slot, const uint8_t* pages, i
 /* Device copy of slot `slot`'s complete results (same layout) and the stream its last writes were enqueued on.   */
 CTD_API int ctd_device_arena(ctd_handle* h, int32_t slot, void** base, void** post_stream);
 
+/* ---- text-line crops for OCR (SURVEY 8f row f4) -----------------------------------------------------------------
+ * `TextBlock.get_transformed_region(img, idx, textheight)` (utils/textblock.py:162-194) for many lines in one call:
+ * quad expansion by font_size / 3 and clip to [0, im_w] x [0, im_h] (flags bit CTD_REGION_EXPAND), aspect ratio of
+ * the quad's mid-lines, output size (h = int(textheight), w = round-half-even(textheight / ratio) for horizontal lines;
+ * w = int(textheight), h = round(textheight * ratio) for vertical ones), `cv2.findHomography(src, dst, RANSAC, 5.0)`
+ * (4 points: normalised DLT), `cv2.warpPerspective(img, M, (w, h))` (INTER_LINEAR, BORDER_CONSTANT 0, OpenCV's
+ * fixed-point arithmetic) and, for vertical lines, `cv2.rotate(.., ROTATE_90_COUNTERCLOCKWISE)`.  Bit-exact with
+ * OpenCV 4.x; csrc/regions.cu.  A w or h of 0 gives a crop of the page's size (OpenCV's empty dsize);
+ * a line the reference cannot crop gets a non-zero status and no bytes.                                         */
+#define CTD_REGION_EXPAND 1          /* flags bit 0: language 'eng', or 'unknown' and not vertical (textblock.py:168) */
+#define CTD_REGION_VERTICAL 2        /* flags bit 1: TextBlock.vertical                                            */
+#define CTD_REGION_OK 0
+#define CTD_REGION_E_RATIO 1         /* ratio 0, inf or nan: the reference's round() raises OverflowError / ValueError */
+#define CTD_REGION_E_HOMOGRAPHY 2    /* w or h is 1, or the quad has no extent along x or y: findHomography returns
+                                        None and warpPerspective raises cv2.error                                   */
+#define CTD_REGION_E_SIZE 3          /* the crop would exceed 2^31 bytes                                            */
+typedef struct ctd_region {
+  int32_t status;        /* CTD_REGION_*                                                                     */
+  int32_t out_h, out_w;  /* crop shape after the rotation of vertical lines (times `channels` bytes per pixel) */
+  int32_t w, h;          /* the reference's w, h (dst corners (w-1, h-1))                                    */
+  int32_t reserved;
+  size_t offset;         /* byte offset of the crop in the packed output (crops follow each other, no padding) */
+  size_t bytes;          /* out_h * out_w * channels (0 when status != 0)                                    */
+  double M[9];           /* forward homography, row-major: filled by ctd_transform_regions                   */
+} ctd_region;
+/* Host-only planning (no handle, thread-safe): quads f64 [n][4][2], flags i32 [n], font_size f64 [n] -> regions[n]
+ * (status, shape, offset, bytes; M = 0) and *total_bytes of the packed output.  CTD_E_INVALID for channels
+ * not in {1, 3}.                                                                                                 */
+CTD_API int ctd_plan_regions(const double* quads, const int32_t* flags, const double* font_size, int32_t n, int32_t im_w,
+                             int32_t im_h, int32_t channels, double textheight, ctd_region* regions, size_t* total_bytes);
+/* All crops of one page in one call on the handle's stream (blocking): img u8 [ih][iw][channels] (HOST, uploaded once
+ * into the handle's grow-on-demand scratch, or with img_on_device != 0 a DEVICE pointer, read in place); out receives
+ * the packed crops (HOST, or with out_on_device != 0 a DEVICE pointer) and must hold the planned total
+ * (CTD_E_CAPACITY otherwise, with regions[] planned).  regions[] as ctd_plan_regions plus the forward M of every
+ * line with status 0.                                                                                            */
+CTD_API int ctd_transform_regions(ctd_handle* h, const uint8_t* img, int32_t ih, int32_t iw, int32_t channels,
+                                  int32_t img_on_device, const double* quads, const int32_t* flags, const double* font_size,
+                                  int32_t n, double textheight, ctd_region* regions, uint8_t* out, int32_t out_on_device,
+                                  size_t out_bytes);
+
 /* utils/yolov5_utils.py:124-218 on a caller-supplied prediction tensor (HOST f32
  * [rows][5+nc]); output as ctd_get_detections for one page.                                */
 CTD_API int ctd_nms(ctd_handle* h, const float* pred, int32_t rows, float conf_thresh, float iou_thresh, float* det,
